@@ -10,10 +10,10 @@ DxD inversions + constants + E-step operand (one device kernel; option "finalize
 / GMM_FINALIZE=host: on the host with one D2H and one H2D) -> E-step (responsibilities
 + log-likelihood), on the synthetic workload of BASELINE.json config 3
 (N=10M, D=24, K=64; config 4 shards the same 10M events over N GPUs = strong
-scaling).  `value` is measured with the events resident in HBM: a block of exactly
-K steps is timed (barrier + synchronize on both sides, device clock, max over
-ranks); the block is repeated `--repeats` times and the MEDIAN block is reported
-(`blocks_ms_per_step` lists all of them).  `e2e` is measured through the C ABI from
+scaling).  `value` is measured with the events resident in HBM: exactly K steps are
+timed, split as evenly as possible into at most `--repeats` blocks (barrier +
+synchronize on both sides, device clock, max over ranks); the MEDIAN block time per
+step is reported (`blocks_ms_per_step` lists all of them).  `e2e` is measured through the C ABI from
 HOST buffers (pinned events H2D, parameters H2D, initial E-step, the K steps,
 parameters + log-likelihood D2H all inside the timed region: one upload per K steps).
 
@@ -22,6 +22,11 @@ dense BF16/FP16 peak — the pipe the kernel's kind::f16 MMAs run on), `cpu_base
 sequential-EM CPU port on the host cores, median of 3), `reference_gpu` (the UNMODIFIED
 reference program compiled for sm_100a, oracle/_ref/gaussianMPI_ref_perf, run on this GPU at
 config 2 and config 3) and `config5` (the model-order-reduction loop K=128 -> 16, gmm_fit).
+
+`--dump-outputs DIR` writes, right after the timed steps, what the last of them computed
+(rank 0: parameters, log-likelihood, memberships of a fixed seeded sample of its events) as
+DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be
+compared array for array.
 
 `--impl reference` times the reference's algorithm on the host cores (the
 sequential-EM CPU port in oracle/, FP32, OpenMP over the physical cores) on a bounded
@@ -245,12 +250,43 @@ def run_reference_gpu(pkg, workload, device, iters=3):
                     f"ENABLE_OUTPUT 0, MIN=MAX_ITERS={iters}, 1 GPU, {workload}: N={N} D={D} K={K}; its own profile_t timers (gaussian.cu:967)")
 
 
+def block_sizes(steps, repeats):
+    """`steps` timed steps split as evenly as possible into at most `repeats` blocks (at least one step each)."""
+    n = max(1, min(repeats, steps))
+    return [steps // n + (1 if i < steps % n else 0) for i in range(n)]
+
+
+DUMP_MEMB_BYTES = 32 << 20         # memberships written by --dump-outputs: 131072 events at K = 64
+
+
+def dump_outputs(pkg, eng, K, D, n, ll, out_dir):
+    """Write what a caller of gmm_em_iterations receives after the last timed step (gmm_get_clusters with memberships,
+    and the log-likelihood) as <out_dir>/<name>.npy.  Memberships [K][n] larger than DUMP_MEMB_BYTES are sampled: a
+    fixed, seeded, sorted choice of events, whose indices are written next to them (35 MB in all at config 3)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cl = eng.get_clusters(K, out=pkg.Clusters(K, D, n), with_memberships=True)
+    arrays = {f: getattr(cl, f)[:K] for f in pkg.Clusters.FIELDS}
+    arrays["loglik"] = np.array([ll], np.float64)
+    m = DUMP_MEMB_BYTES // (4 * K)
+    if n > m:
+        idx = np.sort(np.random.default_rng(pkg.synth.SEED).choice(n, m, replace=False))
+        arrays["memberships"] = cl.memberships[:K, idx]
+        arrays["memberships_events"] = idx.astype(np.float64)
+    else:
+        arrays["memberships"] = cl.memberships[:K]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    return dict(dir=out_dir, arrays=sorted(arrays), bytes=int(sum(a.nbytes for a in arrays.values())),
+                memberships_events=int(arrays["memberships"].shape[1]))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--repeats", type=int, default=5, help="timed blocks of --steps iterations; the median block is reported")
+    ap.add_argument("--repeats", type=int, default=5,
+                    help="timed blocks the --steps iterations are split into; the median time per step of a block is reported")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "cpu-worker"])
     ap.add_argument("--workload", default=os.environ.get("GMM_BENCH_WORKLOAD", "c3"), choices=list(WORKLOADS))
     ap.add_argument("--path", default=os.environ.get("GMM_BENCH_PATH", "auto"), choices=["auto", "simt", "tensor"])
@@ -260,6 +296,9 @@ def main():
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip the reference-on-B200 runs (config 2 and 3)")
     ap.add_argument("--c5-iters", type=int, default=int(os.environ.get("GMM_BENCH_C5_ITERS", "2")),
                     help="EM iterations per model order of the config-5 measurement (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the parameters, log-likelihood and (sampled) memberships they computed "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "cpu-worker":
         return cpu_worker(args)
@@ -351,28 +390,31 @@ def main():
     if rank == 0:
         sampler.wait_ready()
     eng.profile(reset=True)
-    blocks, walls = [], []
+    blocks, walls = [], []                               # seconds per step of each timed block
     m0 = None
     ll = 0.0
-    for _ in range(max(1, args.repeats)):
+    for n_block in block_sizes(args.steps, args.repeats):
         barrier()
         if m0 is None:
             m0 = sampler.mark()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         t0 = time.perf_counter()
-        ll = eng.em_iterations(K, args.steps)            # exactly `steps` iterations; returns after a stream sync
+        ll = eng.em_iterations(K, n_block)               # exactly `n_block` iterations; returns after a stream sync
         ev1.record()
         torch.cuda.synchronize()
-        walls.append(time.perf_counter() - t0)
-        blocks.append(max_over_ranks(ev0.elapsed_time(ev1) * 1e-3))   # device clock around the block, max over ranks
+        walls.append((time.perf_counter() - t0) / n_block)
+        blocks.append(max_over_ranks(ev0.elapsed_time(ev1) * 1e-3) / n_block)   # device clock around the block, max over ranks
     m1 = sampler.mark()
     barrier()
     clocks = sampler.stop(m0, m1) if rank == 0 else None
     dt = float(np.median(blocks))
     dt_wall = float(np.median(walls))
     prof = eng.profile()
-    value = args.steps / dt
+    value = 1.0 / dt
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(pkg, eng, K, D, count, ll, args.dump_outputs)
 
     # ---- end to end from host buffers: e2e ----
     e2e = None
@@ -482,7 +524,7 @@ def main():
         reference_gpu = {w: run_reference_gpu(pkg, w, local_rank) for w in (("c2", "c3") if args.workload == "c3" else (args.workload,))}
 
     line = dict(metric=metric, value=value, unit="it/s", n_gpus=world, steps=args.steps, warmup=args.warmup,
-                ms_per_step=dt * 1e3 / args.steps, higher_is_better=True, scaling=args.scaling, vs_baseline=None,
+                ms_per_step=dt * 1e3, higher_is_better=True, scaling=args.scaling, vs_baseline=None,
                 dtype="f32", data="synthetic",
                 config=dict(workload=f"{args.workload}: N={N} D={D} K={K} Gaussian blobs (seed {pkg.synth.SEED}), "
                                      f"{count} events on rank 0", path=args.path, l2="inputs (X 0.96 GB + memberships 2.56 GB at c3) exceed the 126 MB L2",
@@ -491,13 +533,13 @@ def main():
                             arithmetic=("fp32 data and results; tensor path: fp16 hi/lo split operands, fp32 TMEM accumulation, fp64 "
                                         "statistics reduction and finalisation" if args.path != "simt" else
                                         "fp32 E-step, fp64 M-step statistics and host finalisation"),
-                            timing=f"median of {len(blocks)} timed blocks of {args.steps} steps each"),
+                            timing=f"{args.steps} timed steps in {len(blocks)} blocks; median over the blocks of the time per step"),
                 clocks=clocks, e2e=e2e, gpu_launches=launches_per_step * args.steps, roofline=roofline, roofline_mstep=roofline_mstep,
                 phases_ms_per_step=dict(estep=estep_ms, mstep=mstep_ms, constants_host=prof["constants_host_ms"] / n_it,
                                         allreduce=prof["allreduce_ms"] / n_it, upload=prof["upload_ms"] / n_it),
-                blocks_ms_per_step=[b * 1e3 / args.steps for b in blocks],
-                loglik=ll, wall_ms_per_step=dt_wall * 1e3 / args.steps, cpu_baseline=cpu_baseline, reference_gpu=reference_gpu,
-                config5=config5, comm=dict(rank=r_, nranks=n_))
+                blocks_ms_per_step=[b * 1e3 for b in blocks],
+                loglik=ll, wall_ms_per_step=dt_wall * 1e3, cpu_baseline=cpu_baseline, reference_gpu=reference_gpu,
+                config5=config5, comm=dict(rank=r_, nranks=n_), dump_outputs=dumped)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

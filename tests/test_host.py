@@ -4,6 +4,7 @@ Rissanen, order reduction) against the oracle, file formats, CLI argument rules.
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -37,12 +38,23 @@ def test_no_oracle_in_product(pkg):
 
 
 def test_compute_fails_loudly_without_gpu(pkg):
-    from conftest import have_gpu
-    if have_gpu():
-        pytest.skip("GPU present")
-    with pytest.raises(pkg.GmmError) as ei:
-        pkg.Engine(np.zeros((16, 4), np.float32), 2)
-    assert ei.value.code == 4
+    """No visible GPU (none installed, or CUDA_VISIBLE_DEVICES empty): creating a context raises GMM_ERR_CUDA. Run in a
+    child process with the devices hidden, so that a machine with a GPU checks it too."""
+    code = """if True:
+        import sys
+        sys.path.insert(0, sys.argv[1])
+        import numpy as np
+        import __graft_entry__ as entry
+        pkg = entry.load_package()
+        try:
+            pkg.Engine(np.zeros((16, 4), np.float32), 2)
+        except pkg.GmmError as ex:
+            print("GmmError", ex.code)
+    """
+    r = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert r.stdout.strip().splitlines()[-1] == "GmmError 4", r.stdout + r.stderr
 
 
 def test_host_invert(pkg, oracle64):
