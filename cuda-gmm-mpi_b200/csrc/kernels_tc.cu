@@ -913,7 +913,6 @@ struct TcState {
     float* d_den = nullptr;          // [memb_pitch] running / total log-denominator per event (Kmax > 64 only)
     int e_ck_len = 0;                // Kmax rounded up to whole passes of 64
     int e_NG = 0;
-    int host_threads = 8;
     // cudaFuncAttributeMaxDynamicSharedMemorySize is per device: the "already set" flags live with the (per-device) state
     bool attr_estep = false, attr_mstep = false;
     double h_shift[GMM_MAX_DIMENSIONS] = {0}, h_scale[GMM_MAX_DIMENSIONS] = {0};
@@ -1014,7 +1013,6 @@ int tc_create(TcState** out, const float* d_x_aos, const float* d_x_soa, int n, 
     return GMM_OK;
 }
 
-void tc_set_host_threads(TcState* t, int n) { if (t) t->host_threads = n < 1 ? 1 : n; }
 bool tc_mstep_ready(const TcState* t) { return t && t->maps_ok && t->have_shift && t->mstep_ready; }
 bool tc_estep_range_ok(const TcState* t) {
     if (!t || !t->have_shift) return false;
@@ -1248,21 +1246,6 @@ int tc_params_commit(TcState* t, int K, int bad, cudaStream_t stream) {
     TC_CUDA_TRY(cudaEventRecord(t->ev_h2d, stream));
     t->h2d_pending = true;
     return GMM_OK;
-}
-
-
-int tc_upload_params(TcState* t, const clusters_t* host, int K, cudaStream_t stream) {
-    if (int rc = tc_params_begin(t, K, stream)) return rc;
-    const int kp = tc_params_padded(t, K);
-    const int nt = t->host_threads;
-    int bad = 0;
-    (void)nt;
-#pragma omp parallel for schedule(static) num_threads(nt) reduction(max : bad) if (nt > 1 && K >= 8)
-    for (int k = 0; k < kp; k++) {
-        const int b = tc_params_cluster(t, host, k, K);
-        bad = b > bad ? b : bad;
-    }
-    return tc_params_commit(t, K, bad, stream);
 }
 
 // ===========================================================================

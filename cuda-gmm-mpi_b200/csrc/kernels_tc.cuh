@@ -16,7 +16,6 @@ bool tc_estep_supported(int D, int K);
 int  tc_create(TcState** out, const float* d_x_aos, const float* d_x_soa, int n, int D, int Kmax, float* d_memb, size_t memb_pitch,
                int num_sms, cudaStream_t stream);
 void tc_destroy(TcState*);
-void tc_set_host_threads(TcState*, int n);
 // Centre/scale used inside the tensor kernels: z = (x - shift) * inv_scale, both rounded to
 // float; `shift` is updated in place to the float-rounded values actually used.  xmin / xmax: per-dimension extremes
 // of the WHOLE data set (all ranks): they fix the power-of-two quanta of the M-step's fixed-point operand parts.
@@ -26,10 +25,10 @@ int  tc_set_shift_scale(TcState*, double* shift, const double* scale, const doub
 bool tc_mstep_ready(const TcState*);
 // False when an event lies beyond 2^14 global standard deviations (its standardised coordinates would overflow FP16).
 bool tc_estep_range_ok(const TcState*);
-int  tc_upload_params(TcState*, const clusters_t* host, int K, cudaStream_t stream);
-// The same in three steps, so that the caller can fuse the per-cluster work with its own per-cluster
-// finalisation in ONE parallel loop: begin (serial), cluster k in [0, tc_params_padded) (independent, thread
-// safe; returns 0 or a defect code to be max-reduced), commit (serial: error report or H2D of the operand).
+// The tensor E-step operand of the host parameters in three steps, so that the caller can fuse the per-cluster work
+// with its own per-cluster finalisation in ONE parallel loop: begin (serial), cluster k in [0, tc_params_padded)
+// (independent, thread safe; returns 0 or a defect code to be max-reduced), commit (serial: error report or H2D of
+// the operand).
 int  tc_params_begin(TcState*, int K, cudaStream_t stream);
 int  tc_params_padded(const TcState*, int K);
 int  tc_params_cluster(TcState*, const clusters_t* host, int k, int K);
